@@ -164,6 +164,21 @@ def cpu_reference_step(frames, threads=None):
     return step, kind, threads
 
 
+DUMP_SAMPLE = 1 << 23          # elements kept of an output larger than this (32 MB): a fixed seeded choice of indices, the same in every run
+
+
+def dump_outputs(out_dir, **arrays):
+    """Writes each array as out_dir/<name>.npy in float32.  An array above DUMP_SAMPLE elements is flattened and sampled at DUMP_SAMPLE
+    sorted indices drawn from seed 0, so two runs sample the same elements and the dump of the synthesis step stays below 64 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+
+
 def run_reference(args):
     """--impl reference: the reference's own implementation of the path on the host cores — the unmodified reference SynthesisNetwork with
     custom CUDA disabled — on a bounded sample (8 of the 32 frames of a step) with the requested steps / warm-up (shortened only if the
@@ -524,7 +539,13 @@ def main():
     ap.add_argument('--ref-frames', type=int, default=8, help='--impl reference: frames per sampled CPU step (of the 32 of a step)')
     ap.add_argument('--workload', default='synthesis', choices=['synthesis', 'gd_step', 'synthesis_fwd', 'full_loop'],
                     help="synthesis = BASELINE metric (256x256 SynthesisNetwork fwd+bwd, configs[1] batch); gd_step = configs[2] (G+D training step, no reg)")
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='synthesis workload, one GPU: after the timed steps run the timed step once more on the starting parameters and the same '
+                         'inputs and write what it computes (image, loss, d loss / d ws, d loss / d parameters) as DIR/<name>.npy in float32, '
+                         'for comparing two builds output for output')
     args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != 'b200' or args.workload != 'synthesis'):
+        ap.error('--dump-outputs is implemented for the default synthesis workload of the b200 implementation')
     if args.impl == 'reference':
         return run_reference(args)
     if args.workload == 'gd_step':
@@ -567,6 +588,9 @@ def main():
     state.broadcast(0)                         # ... and rank 0's parameters are broadcast like the reference's "Distribute across GPUs" (training_loop.py:215-232)
     bucket = dict(armed=False)                 # whether the step being built carries its collectives (stylegan_v_b200/optim.py: begin / finish_backward)
     opt = None if args.no_optimizer else FusedAdamEMA(state, lr=0.0025, betas=(0.0, 0.99), eps=1e-8)
+    if args.dump_outputs is not None:
+        assert world == 1, '--dump-outputs runs on one GPU'
+        p0 = state.param.clone()               # the starting parameters: what the dumped step is computed from
     torch.manual_seed(1 + rank)                # per-rank latents (each rank works on its own 32 frames)
     N = FRAMES_PER_GPU
     L = net.motion_encoder.traj_len()
@@ -577,6 +601,7 @@ def main():
     d_ws, d_t, d_mz = h_ws.to(dev), h_t.to(dev), h_mz.to(dev)
     dimg = torch.randn(N, 3, RES, RES, device=dev)
     h_out = torch.zeros(1).pin_memory()
+    last = {}                                  # image, loss and ws (.grad) of the latest step (graph outputs are rewritten by every replay)
 
     def step_compute(ws, t, mz):
         if opt is None:
@@ -589,6 +614,7 @@ def main():
         loss.backward()
         if bucket['armed']:
             state.finish_backward()            # waits for the conv-weight bucket (stream-level, capturable), reduces the rest: affines, biases, motion encoder
+        last.update(img=img, loss=loss, ws=ws)
         return loss
 
     # The step (about 670 kernel launches: forward + backward of 20 fused layers) is captured ONCE into a CUDA graph and replayed:
@@ -701,6 +727,23 @@ def main():
         h_out.copy_(loss.detach().reshape(1), non_blocking=True)
     ms_e2e, _ = timed(e2e_step, args.steps, 1)
     clocks = sampler.stop() if rank == 0 else None      # sampled across both timed regions (device-resident and end-to-end)
+    if args.dump_outputs is not None:
+        # Every timed step updates the parameters, and the atomic reductions of the kernels make each gradient exact only up to rounding; over
+        # many Adam steps on this unbounded loss those differences grow, so the state the timed steps end in is not the same in every run.  The
+        # dump is the timed step (the same graph, or the same eager launches) evaluated once more on the starting parameters and the same
+        # inputs: the same in every run up to rounding.  The parameters the timed steps reached are put back afterwards.
+        p_now = state.param.clone()
+        state.param.copy_(p0)
+        state.zero_grad()
+        if graph is not None:
+            graph.replay()
+        else:
+            with precision.precision(args.precision):
+                step_compute(d_ws.detach(), d_t, d_mz)
+        dump_outputs(args.dump_outputs, img=last['img'], loss=last['loss'], ws_grad=last['ws'].grad, param_grad=state.grad)
+        state.param.copy_(p_now)
+        state.zero_grad()
+        del p0, p_now
 
     # (3) the same step in the other arithmetic mode, beside the headline (the reference trains with allow_tf32 = False, training_loop.py:141-142:
     #     tf32x3 is the fp32-grade counterpart; tf32 is the north_star's TF32 tensor-core arithmetic)

@@ -371,6 +371,8 @@ def gen_mixed_precision(ref):
                img_eval=img_eval.numpy(), img_eval_b1=img_eval_b1.numpy(), d_ws=grads[0].numpy())
     for n, a in zip(keep, grads[1:]):
         out['g:' + n] = a.numpy()
+    out['meta'] = np.frombuffer(json.dumps(dict(G=TINY, num_fp16_res=2, conv_clamp=256)).encode(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(OUT, 'mixed_precision_g_tiny.npz'), **out)          # G and D in two files: each stays below 1 MB
     # discriminator
     d = TINY_D
     dcfg = ref_loader.to_cfg(dict(sampling=dict(num_frames_per_video=3, max_num_frames=d['max_num_frames'], type='random'),
@@ -382,12 +384,18 @@ def gen_mixed_precision(ref):
     dimg_in = torch.randn(6, 3, 32, 32, generator=g).requires_grad_(True)
     dt = torch.tensor([[0.0, 5.0, 9.0], [100.0, 101.0, 131.0]])
     D.train()
+    # the time-difference embedding (1024 rows) is read only at the differences of dt: zero the rows this clip never reads (their
+    # gradient is zero), which leaves every output unchanged and keeps the file small
+    emb = D.time_encoder.const_embed.weight
+    used, = torch.autograd.grad(D(dimg_in, torch.zeros(2, 0), dt)['image_logits'].sum(), [emb])
+    with torch.no_grad():
+        emb[used.abs().sum(1) == 0] = 0
     logits = D(dimg_in, torch.zeros(2, 0), dt)['image_logits']
     gin, gw = torch.autograd.grad(logits.sum(), [dimg_in, D.b8.conv0.weight])
-    out.update({'d:' + k: v.detach().numpy().copy() for k, v in D.state_dict().items()})
+    out = {'d:' + k: v.detach().numpy().copy() for k, v in D.state_dict().items()}
     out.update(d_img=dimg_in.detach().numpy(), d_t=dt.numpy(), d_logits=logits.detach().numpy(), d_gin=gin.numpy(), d_gw_b8_conv0=gw.numpy())
-    out['meta'] = np.frombuffer(json.dumps(dict(G=TINY, D=TINY_D, num_fp16_res=2, conv_clamp=256)).encode(), dtype=np.uint8)
-    np.savez_compressed(os.path.join(OUT, 'mixed_precision_tiny.npz'), **out)
+    out['meta'] = np.frombuffer(json.dumps(dict(D=TINY_D, num_fp16_res=2, conv_clamp=256)).encode(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(OUT, 'mixed_precision_d_tiny.npz'), **out)
 
 
 AUG_CASES = [
@@ -485,6 +493,186 @@ def gen_loss_phases(ref):
     np.savez_compressed(os.path.join(OUT, 'loss_phases_tiny.npz'), **out)
 
 
+NET64_G = dict(img_resolution=64, w_dim=64, channel_base=4096, channel_max=64, motion_z_dim=32, motion_v_dim=32, time_enc_dim=32)
+NET64_D = dict(img_resolution=64, channel_base=4096, channel_max=64, num_frames_per_video=3, max_num_frames=1024, concat_res=16,
+               num_frames_div_factor=2, mbstd_group_size=2, mapping_layers=2)
+NET64_G_NAMES = ['synthesis.b64.conv1.weight', 'synthesis.b32.conv0.weight', 'synthesis.b8.conv1.weight', 'synthesis.b64.torgb.weight',
+                 'synthesis.b16.conv1.bias', 'mapping.fc1.weight', 'synthesis.motion_encoder.conv.0.weight']
+NET64_D_NAMES = ['b64.conv0.weight', 'b64.conv1.weight', 'b32.skip.weight', 'b16.conv0.weight', 'b4.conv.weight', 'b4.out.weight', 'b64.fromrgb.weight']
+LOSS32_G = dict(img_resolution=32, w_dim=64, channel_base=2048, channel_max=64, motion_z_dim=32, motion_v_dim=32, time_enc_dim=32)
+LOSS32_D = dict(NET64_D, img_resolution=32, channel_base=2048)
+SAMPLE = 4096
+
+
+def seeded_modules(gk, dk):
+    """The project's own Generator / Discriminator for the configs gk / dk, initialised from torch seed 0, every bias (but the affines')
+    drawn from seed 1 in name order.  Goldens minted on these parameters do not have to store them."""
+    from stylegan_v_b200.networks import Generator, Discriminator
+    cfg = sr.SynthesisConfig(**gk)
+    torch.manual_seed(0)
+    G = Generator.from_reference_cfg(cfg.reference_generator_cfg(), img_resolution=cfg.img_resolution, channel_base=cfg.channel_base,
+                                     channel_max=cfg.channel_max, mapping_layers=2)
+    D = Discriminator.from_reference_cfg(d_cfg(dk), img_resolution=dk['img_resolution'], channel_base=dk['channel_base'],
+                                         channel_max=dk['channel_max'], mbstd_group_size=dk['mbstd_group_size'], mapping_layers=dk['mapping_layers'])
+    g = torch.Generator().manual_seed(1)
+    with torch.no_grad():
+        for m in (G, D):
+            for n, p in sorted(m.named_parameters()):
+                if n.endswith('.bias') and 'affine' not in n:
+                    p.copy_(torch.randn(p.shape, generator=g) * 0.1)
+    return G, D
+
+
+def d_cfg(dk):
+    return dict(sampling=dict(num_frames_per_video=dk['num_frames_per_video'], max_num_frames=dk['max_num_frames'], type='random'),
+                concat_res=dk['concat_res'], num_frames_div_factor=dk['num_frames_div_factor'], dummy_c=False)
+
+
+def param_sum(G, D):
+    """sum |p| over both state dicts in float64: tells a changed initialisation of the project's modules from a changed kernel."""
+    return float(sum(v.double().abs().sum() for m in (G, D) for v in m.state_dict().values()))
+
+
+def sample(a, dtype=np.float64):
+    """A fixed sample of SAMPLE elements of a (all of it when smaller)."""
+    a = a.detach().double().cpu().contiguous().reshape(-1).numpy().astype(dtype)
+    if a.size <= SAMPLE:
+        return a
+    return a[np.sort(np.random.default_rng(a.size).choice(a.size, SAMPLE, replace=False))]
+
+
+def reference_gd(ref, gk, dk, Gp, Dp):
+    """The reference Generator / Discriminator for gk / dk carrying the parameters of the project's modules Gp / Dp."""
+    cfg = sr.SynthesisConfig(**gk)
+    G = ref.networks.Generator(c_dim=0, w_dim=cfg.w_dim, img_resolution=cfg.img_resolution, img_channels=3, cfg=ref_loader.to_cfg(cfg.reference_generator_cfg()),
+                               mapping_kwargs=dict(num_layers=2), synthesis_kwargs=dict(channel_base=cfg.channel_base, channel_max=cfg.channel_max)).train()
+    D = ref.networks.Discriminator(c_dim=0, img_resolution=dk['img_resolution'], img_channels=3, channel_base=dk['channel_base'], channel_max=dk['channel_max'],
+                                   cfg=ref_loader.to_cfg(d_cfg(dk)), mapping_kwargs=dict(num_layers=dk['mapping_layers']),
+                                   epilogue_kwargs=dict(mbstd_group_size=dk['mbstd_group_size'])).train()
+    load_parameters(G, Gp)
+    load_parameters(D, Dp)
+    return G, D
+
+
+def load_parameters(ref_module, module):
+    """Copies the parameters of the project's module into the reference module; the reference keeps its own buffers (FIR filters,
+    frequencies, ...), so that those are compared too."""
+    missing, unexpected = ref_module.load_state_dict(dict(module.named_parameters()), strict=False)
+    buffers = dict(ref_module.named_buffers())
+    assert not unexpected and all(k in buffers for k in missing), (unexpected, [k for k in missing if k not in buffers])
+
+
+def gen_networks_64(ref):
+    """The reference Generator + Discriminator (networks.py:370-673) at 64x64, channel_max 64, on CPU (its impl='ref' ops), on the
+    parameters of the project's own modules (`seeded_modules`): image, logits of D on the generated clip, and the gradients of the
+    softplus(-logits) loss w.r.t. a set of G and D weights.  tests/test_zz_reference_on_dropin_gpu.py runs the same modules on cuda:0."""
+    cfg = sr.SynthesisConfig(**NET64_G)
+    Gp, Dp = seeded_modules(NET64_G, NET64_D)
+    G, D = reference_gd(ref, NET64_G, NET64_D, Gp, Dp)
+    g = torch.Generator().manual_seed(2)
+    B = 2
+    z = torch.randn(B, cfg.w_dim, generator=g)
+    t = torch.tensor([[0.0, 5.0, 9.0], [100.0, 116.5, 131.0]])
+    c = torch.zeros(B, 0)
+    mz = torch.randn(B, sr.max_traj_len(cfg, float(t.max())), cfg.motion_z_dim, generator=g)
+    img = G(z, c, t, motion_z=mz)
+    logits = D(img, c, t)['image_logits']
+    torch.nn.functional.softplus(-logits).mean().backward()
+    gp, dp = dict(G.named_parameters()), dict(D.named_parameters())
+    out = dict(z=z.numpy(), t=t.numpy(), motion_z=mz.numpy(), img=img.detach().numpy(), logits=logits.detach().numpy(),
+               param_sum=np.float64(param_sum(Gp, Dp)))
+    out.update({'G:' + n: sample(gp[n].grad) for n in NET64_G_NAMES})
+    out.update({'D:' + n: sample(dp[n].grad) for n in NET64_D_NAMES})
+    out['meta'] = np.frombuffer(json.dumps(dict(G=NET64_G, D=NET64_D, sample=SAMPLE)).encode(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(OUT, 'networks_64.npz'), **out)
+
+
+def gen_loss_phases_32(ref):
+    """The reference's StyleGAN2Loss.accumulate_gradients (loss.py:73-173) for Gmain, Dmain and Dreg (R1, gain 16) at 32x32, channel_max 64,
+    on the parameters of the project's own modules (`seeded_modules`), CPU: a fixed float32 sample of every weight gradient of at least 64
+    elements.  The motion noise the reference draws inside G (motion.py:83) comes from one CPU generator reseeded per phase and is stored,
+    so that a CUDA evaluation can be fed the same draws."""
+    Gp, Dp = seeded_modules(LOSS32_G, LOSS32_D)
+    G, D = reference_gd(ref, LOSS32_G, LOSS32_D, Gp, Dp)
+    loss = ref.loss.StyleGAN2Loss(cfg=None, device=torch.device('cpu'), G_mapping=G.mapping, G_synthesis=G.synthesis, D=D,
+                                  style_mixing_prob=0.0, r1_gamma=0.5, pl_weight=0.0)
+    g = torch.Generator().manual_seed(2)
+    B, Fr, R = 2, 3, LOSS32_G['img_resolution']
+    real = torch.randn(B, Fr, 3, R, R, generator=g).clamp(-1, 1)
+    real_t = torch.tensor([[0.0, 4.0, 20.0], [30.0, 31.0, 33.0]])
+    gen_t = torch.tensor([[2.0, 10.0, 11.0], [500.0, 516.0, 530.0]])
+    z = torch.randn(B, LOSS32_G['w_dim'], generator=g)
+    c = torch.zeros(B, 0)
+    out = dict(real=real.numpy(), real_t=real_t.numpy(), gen_t=gen_t.numpy(), z=z.numpy(), param_sum=np.float64(param_sum(Gp, Dp)))
+    randn, draws, gen = torch.randn, [], torch.Generator()
+
+    def recorded_randn(*size, **kw):
+        kw.pop('generator', None)
+        x = randn(*size, generator=gen, **kw)
+        draws.append(x)
+        return x
+    w0 = G.mapping.w_avg.clone()
+    torch.randn = recorded_randn
+    try:
+        for phase, module, gain in [('Gmain', G, 1), ('Dmain', D, 1), ('Dreg', D, 16)]:
+            G.requires_grad_(module is G); D.requires_grad_(module is D)
+            for p in module.parameters():
+                p.grad = None
+            gen.manual_seed(100)
+            draws.clear()
+            loss.accumulate_gradients(phase=phase, real_img=real, real_c=c, real_t=real_t, gen_z=z, gen_c=c, gen_t=gen_t, sync=True, gain=gain)
+            G.mapping.w_avg.copy_(w0)
+            assert len(draws) == (0 if phase == 'Dreg' else 1), (phase, len(draws))
+            if draws:
+                out[f'motion_z:{phase}'] = draws[0].numpy()
+            for n, p in module.named_parameters():
+                if p.grad is not None and p.grad.numel() >= 64 and not n.endswith('bias'):
+                    out[f'{phase}:{n}'] = sample(p.grad, np.float32)
+    finally:
+        torch.randn = randn
+    out['meta'] = np.frombuffer(json.dumps(dict(G=LOSS32_G, D=LOSS32_D, r1_gamma=0.5, sample=SAMPLE)).encode(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(OUT, 'loss_phases_32.npz'), **out)
+
+
+SIGNATURES = {'upfirdn2d': ['setup_filter', 'upfirdn2d', 'filter2d', 'upsample2d', 'downsample2d', '_parse_padding', '_get_filter_size'],
+              'bias_act': ['bias_act'], 'conv2d_resample': ['conv2d_resample'], 'conv2d_gradfix': ['conv2d', 'conv_transpose2d', 'no_weight_gradients'],
+              'fma': ['fma']}
+
+
+def gen_signatures(ref):
+    """The call signatures of the reference's torch_utils.ops functions that the drop-in ops must keep (tests/test_ops_cpu.py).  Functions
+    the reference wraps in misc.profiled_function show `(*args, **kwargs)` and are left out."""
+    import inspect
+    sigs = {}
+    for mod, names in SIGNATURES.items():
+        for n in names:
+            s = str(inspect.signature(getattr(getattr(ref, mod), n)))
+            if s != '(*args, **kwargs)':
+                sigs[f'{mod}.{n}'] = s
+    out = dict(signatures=np.frombuffer(json.dumps(sigs).encode(), dtype=np.uint8), meta=np.frombuffer(b'{}', dtype=np.uint8))
+    np.savez_compressed(os.path.join(OUT, 'reference_signatures.npz'), **out)
+
+
+def gen_config0(ref):
+    """BASELINE configs[0]: the reference SynthesisNetwork at 64x64 (default widths), 1 latent x 1 frame, eval mode, on CPU with its own
+    ops, on the parameters of the project's SynthesisNetwork built from torch seed 0 (tests/test_config0_cpu.py rebuilds them)."""
+    from stylegan_v_b200.synthesis import SynthesisNetwork
+    cfg = sr.SynthesisConfig(img_resolution=64)
+    torch.manual_seed(0)
+    net = SynthesisNetwork.from_config(cfg)
+    S = ref.networks.SynthesisNetwork(w_dim=cfg.w_dim, img_resolution=64, img_channels=3, channel_base=cfg.channel_base, channel_max=cfg.channel_max,
+                                      cfg=ref_loader.to_cfg(cfg.reference_generator_cfg())).eval()
+    load_parameters(S, net)
+    g = torch.Generator().manual_seed(1)
+    ws = torch.randn(1, S.num_ws, cfg.w_dim, generator=g)
+    mz = torch.randn(1, sr.max_traj_len(cfg, 0.0), cfg.motion_z_dim, generator=g)
+    with torch.no_grad():
+        img = S(ws, t=torch.zeros(1, 1), c=torch.zeros(1, 0), motion_z=mz)
+    out = dict(img=img.numpy(), ws=ws.numpy(), mz=mz.numpy(), param_sum=np.float64(sum(float(v.double().abs().sum()) for v in net.state_dict().values())),
+               meta=np.frombuffer(json.dumps(dict(img_resolution=64)).encode(), dtype=np.uint8))
+    np.savez_compressed(os.path.join(OUT, 'config0_64.npz'), **out)
+
+
 def main(only=None):
     os.makedirs(OUT, exist_ok=True)
     ref = ref_loader.load()
@@ -504,6 +692,10 @@ def main(only=None):
     gen_loss_phases(ref)
     gen_mixed_precision(ref)
     gen_augment(ref)
+    gen_networks_64(ref)
+    gen_loss_phases_32(ref)
+    gen_signatures(ref)
+    gen_config0(ref)
     for fn in sorted(os.listdir(OUT)):
         print(fn, os.path.getsize(os.path.join(OUT, fn)))
 

@@ -12,8 +12,6 @@ import pytest
 from conftest import ROOT
 from oracle import ref_loader
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason='reference tree not present')
-
 _WRITE = r'''
 import sys, pickle, numpy as np, torch
 sys.path.insert(0, {root!r})
@@ -62,6 +60,7 @@ assert e1 < 1e-5 and e2 < 1e-5, (e1, e2)
 '''
 
 
+@pytest.mark.skipif(not ref_loader.available(), reason='reference tree not present')
 def test_reference_snapshot_loads_into_native_modules(tmp_path):
     pkl, npz = str(tmp_path / 'network-snapshot.pkl'), str(tmp_path / 'out.npz')
     env = dict(os.environ, OMP_NUM_THREADS='4')

@@ -168,7 +168,7 @@ def test_mixed_precision_mode_vs_reference_golden():
     """num_fp16_res / conv_clamp (the reference's default training precision, train.py:173-174): fp16 activations + clamp 256 in the
     high-resolution blocks of G and D, fp16 pre-normalisation of weights and styles (networks.py:50-52), fused_modconv rule of
     networks.py:232 — on the unfused ops, against the reference run the same way on CPU."""
-    g, meta = load_golden('mixed_precision_tiny.npz')
+    g, meta = load_golden('mixed_precision_g_tiny.npz')
     cfg = sr.SynthesisConfig(**meta['G'])
     kw = dict(w_dim=cfg.w_dim, img_resolution=cfg.img_resolution, channel_base=cfg.channel_base, channel_max=cfg.channel_max,
               motion_z_dim=cfg.motion_z_dim, motion_v_dim=cfg.motion_v_dim, time_enc_dim=cfg.time_enc_dim)
@@ -189,6 +189,7 @@ def test_mixed_precision_mode_vs_reference_golden():
     with torch.no_grad():
         assert rel_err(net(ws, t, motion_z=mz), _t(g['img_eval'])) < 2e-3
         assert rel_err(net(ws[:1], t[:1], motion_z=mz[:1]), _t(g['img_eval_b1'])) < 2e-3
+    g, meta = load_golden('mixed_precision_d_tiny.npz')
     md = meta['D']
     D = Discriminator(c_dim=0, img_resolution=md['img_resolution'], channel_base=md['channel_base'], channel_max=md['channel_max'],
                       num_frames_per_video=md['num_frames_per_video'], max_num_frames=md['max_num_frames'], concat_res=md['concat_res'],

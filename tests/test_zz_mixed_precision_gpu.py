@@ -14,7 +14,7 @@ pytestmark = pytest.mark.gpu
 
 
 def test_mixed_precision_cuda_vs_reference_golden(cuda):
-    g, meta = load_golden('mixed_precision_tiny.npz')
+    g, meta = load_golden('mixed_precision_g_tiny.npz')
     cfg = sr.SynthesisConfig(**meta['G'])
     net = SynthesisNetwork(w_dim=cfg.w_dim, img_resolution=cfg.img_resolution, channel_base=cfg.channel_base, channel_max=cfg.channel_max,
                            motion_z_dim=cfg.motion_z_dim, motion_v_dim=cfg.motion_v_dim, time_enc_dim=cfg.time_enc_dim,
@@ -23,6 +23,7 @@ def test_mixed_precision_cuda_vs_reference_golden(cuda):
     net = net.to(cuda).train()
     img = net(_t(g['ws']).to(cuda), _t(g['t']).to(cuda), motion_z=_t(g['motion_z']).to(cuda))
     assert img.dtype == torch.float32 and rel_err(img, _t(g['img_train'])) < 5e-3
+    g, meta = load_golden('mixed_precision_d_tiny.npz')
     md = meta['D']
     D = Discriminator(c_dim=0, img_resolution=md['img_resolution'], channel_base=md['channel_base'], channel_max=md['channel_max'],
                       num_frames_per_video=md['num_frames_per_video'], max_num_frames=md['max_num_frames'], concat_res=md['concat_res'],

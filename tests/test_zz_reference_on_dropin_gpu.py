@@ -1,116 +1,75 @@
-"""The UNMODIFIED reference Generator / Discriminator (src/training/networks.py:370-673) running on the B200 through the drop-in ops.
+"""Generator + Discriminator and the training-loss phases on the B200 against the reference's own networks (src/training/networks.py:370-673)
+and StyleGAN2Loss (src/training/loss.py:73-173) on the same parameters.
 
-north_star: "keeping the torch_utils.ops plugin API surface so the new kernels drop into the existing Generator/Discriminator unchanged".
-In a fresh interpreter `stylegan_v_b200.install.install_ops()` aliases the op package under the names the reference imports
-(INTEGRATION.md route 1), the reference modules are imported from the reference tree — /root/reference in the build container, the
-hash-verified byte-for-byte copy staged by oracle/stage_ref.py on the GPU box — and the same networks are evaluated
-  (a) on CPU (the reference's `impl='ref'` formulation: BASELINE configs[0] "custom CUDA disabled"), and
-  (b) on cuda:0 with `conv2d_gradfix.enabled = True` like the reference's training loop (training_loop.py:143): FIR / bias_act /
-      contraction kernels of libsgv_b200, in tf32x3 (fp32-grade) and in the default TF32 mode.
-Images, logits and parameter gradients of (b) must match (a); the launch counter proves the library ran.
-Skipped only where no reference tree is available at all."""
+tests/golden/networks_64.npz holds what the reference Generator and Discriminator computed on CPU (its `impl='ref'` ops: BASELINE configs[0]
+"custom CUDA disabled") on the parameters of this project's modules built from fixed seeds (oracle/make_goldens.py, `seeded_modules`):
+the generated clip, D's logits on it, and the gradients of the softplus(-logits) loss w.r.t. a set of G and D weights (a fixed sample of each).
+Here the same modules run on cuda:0 with `conv2d_gradfix.enabled = True` like the reference's training loop (training_loop.py:143): the
+native synthesis path, and the discriminator on the drop-in FIR / bias_act / contraction kernels of libsgv_b200, in tf32x3 (fp32-grade) and
+in the default TF32 mode.  Images, logits and parameter gradients must match the reference; the launch counter proves the library ran.
+tests/golden/loss_phases_32.npz holds the reference loss's Gmain, Dmain and R1 gradients at 32x32 in the same way."""
 import json
-import os
-import subprocess
-import sys
 
+import numpy as np
 import pytest
+import torch
 
-from conftest import ROOT
-from oracle import ref_loader
+from conftest import GOLDEN
+from oracle import make_goldens as M
+from stylegan_v_b200 import train_step as ts
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason='no reference tree (neither /root/reference nor oracle/_ref/pyref)')]
-
-_SCRIPT = r'''
-import sys, json, numpy as np, torch
-sys.path.insert(0, {root!r})
-from stylegan_v_b200.install import install_ops
-install_ops()
-from stylegan_v_b200 import _lib, precision
-from oracle import ref_loader, synthesis_ref as sr
-ref = ref_loader.load()
-import stylegan_v_b200.ops.upfirdn2d as my_up
-assert sys.modules['src.torch_utils.ops.upfirdn2d'] is my_up and ref.networks.upfirdn2d is my_up      # the reference resolved OUR ops
-from stylegan_v_b200.ops import conv2d_gradfix
-torch.backends.cudnn.allow_tf32 = False
-torch.backends.cuda.matmul.allow_tf32 = False
-
-cfg = sr.SynthesisConfig(img_resolution=64, w_dim=64, channel_base=4096, channel_max=64, motion_z_dim=32, motion_v_dim=32, time_enc_dim=32)
-gcfg = ref_loader.to_cfg(cfg.reference_generator_cfg())
-dcfg = ref_loader.to_cfg(dict(sampling=dict(num_frames_per_video=3, max_num_frames=1024, type='random'), concat_res=16, num_frames_div_factor=2, dummy_c=False))
-torch.manual_seed(0)
-G = ref.networks.Generator(c_dim=0, w_dim=cfg.w_dim, img_resolution=64, img_channels=3, cfg=gcfg, mapping_kwargs=dict(num_layers=2),
-                           synthesis_kwargs=dict(channel_base=cfg.channel_base, channel_max=cfg.channel_max)).train()
-D = ref.networks.Discriminator(c_dim=0, img_resolution=64, img_channels=3, channel_base=4096, channel_max=64, cfg=dcfg,
-                               mapping_kwargs=dict(num_layers=2), epilogue_kwargs=dict(mbstd_group_size=2)).train()
-g = torch.Generator().manual_seed(1)
-with torch.no_grad():
-    for n, p in list(G.named_parameters()) + list(D.named_parameters()):
-        if n.endswith('.bias') and 'affine' not in n:
-            p.copy_(torch.randn(p.shape, generator=g) * 0.1)
-B, Fr = 2, 3
-z = torch.randn(B, cfg.w_dim, generator=g)
-t = torch.tensor([[0.0, 5.0, 9.0], [100.0, 116.5, 131.0]])
-c = torch.zeros(B, 0)
-mz = torch.randn(B, sr.max_traj_len(cfg, float(t.max())), cfg.motion_z_dim, generator=g)
-G_NAMES = ['synthesis.b64.conv1.weight', 'synthesis.b32.conv0.weight', 'synthesis.b8.conv1.weight', 'synthesis.b64.torgb.weight', 'synthesis.b16.conv1.bias',
-           'mapping.fc1.weight', 'synthesis.motion_encoder.conv.0.weight']
-D_NAMES = ['b64.conv0.weight', 'b64.conv1.weight', 'b32.skip.weight', 'b16.conv0.weight', 'b4.conv.weight', 'b4.out.weight', 'b64.fromrgb.weight']
+pytestmark = pytest.mark.gpu
 
 
-def run(dev):
-    Gd, Dd = G.to(dev), D.to(dev)
-    for m in (Gd, Dd):
-        m.requires_grad_(True)
-        for p in m.parameters():
-            p.grad = None
-    w0 = Gd.mapping.w_avg.clone()
-    img = Gd(z.to(dev), c.to(dev), t.to(dev), motion_z=mz.to(dev))
-    logits = Dd(img, c.to(dev), t.to(dev))['image_logits']
-    torch.nn.functional.softplus(-logits).mean().backward()
-    Gd.mapping.w_avg.copy_(w0)            # train-mode forward moves the average; keep both evaluations on the same state
-    gp, dp = dict(Gd.named_parameters()), dict(Dd.named_parameters())
-    out = dict(img=img.detach().double().cpu(), logits=logits.detach().double().cpu())
-    out.update({{'G:' + n: gp[n].grad.double().cpu() for n in G_NAMES}})
-    out.update({{'D:' + n: dp[n].grad.double().cpu() for n in D_NAMES}})
-    return out
-
-
-def rel(a, b):
+def _rel(a, b):
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
-cpu = run(torch.device('cpu'))
-dev = torch.device('cuda', 0)
-conv2d_gradfix.enabled = True                                   # training_loop.py:143
-report = dict(ops=ref.networks.upfirdn2d.__name__)
-for mode in ('tf32x3', 'tf32'):
-    n0 = _lib.launch_count()
-    with precision.precision(mode):
-        gpu = run(dev)
-    torch.cuda.synchronize()
-    report[mode] = dict(launches=_lib.launch_count() - n0, **{{k: rel(gpu[k], cpu[k]) for k in cpu}})
-    cosines = {{}}
-    for k in cpu:
-        if k[1] == ':':
-            cosines[k] = float(torch.nn.functional.cosine_similarity(gpu[k].flatten(), cpu[k].flatten(), dim=0))
-    report[mode]['cos'] = cosines
-print('REPORT ' + json.dumps(report))
-'''
+def test_generator_and_discriminator_cuda_vs_reference_golden(cuda):
+    from stylegan_v_b200 import _lib, precision
+    from stylegan_v_b200.ops import conv2d_gradfix
+    g = np.load(f'{GOLDEN}/networks_64.npz')
+    G, D = M.seeded_modules(M.NET64_G, M.NET64_D)
+    assert M.param_sum(G, D) == pytest.approx(float(g['param_sum']), rel=1e-12), \
+        'the seeded initialisation of the modules changed: re-mint tests/golden/networks_64.npz (python -m oracle.make_goldens gen_networks_64)'
+    G, D = G.to(cuda).train(), D.to(cuda).train()
+    z, t, mz = (torch.from_numpy(g[k]).to(cuda) for k in ('z', 't', 'motion_z'))
+    c = torch.zeros(len(z), 0, device=cuda)
+    want = {k: torch.from_numpy(g[k]).double() for k in g.files if k not in ('z', 't', 'motion_z', 'param_sum', 'meta')}
+    w0 = G.mapping.w_avg.clone()
 
+    def run():
+        for m in (G, D):
+            for p in m.parameters():
+                p.grad = None
+        img = G(z, c, t, motion_z=mz)
+        logits = D(img, c, t)['image_logits']
+        torch.nn.functional.softplus(-logits).mean().backward()
+        G.mapping.w_avg.copy_(w0)             # a train-mode forward moves the average; keep both evaluations on the same state
+        gp, dp = dict(G.named_parameters()), dict(D.named_parameters())
+        out = dict(img=img.detach().double().cpu(), logits=logits.detach().double().cpu())
+        out.update({'G:' + n: torch.from_numpy(M.sample(gp[n].grad)) for n in M.NET64_G_NAMES})
+        out.update({'D:' + n: torch.from_numpy(M.sample(dp[n].grad)) for n in M.NET64_D_NAMES})
+        return out
 
-def test_unmodified_reference_generator_and_discriminator_on_dropin_ops(tmp_path):
-    code = _SCRIPT.format(root=ROOT)
-    env = dict(os.environ)
-    env.pop('SGV_PRECISION', None)
-    r = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, env=env, cwd=ROOT, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    line = [ln for ln in r.stdout.splitlines() if ln.startswith('REPORT ')][-1]
-    rep = json.loads(line[len('REPORT '):])
-    assert rep['ops'].startswith('stylegan_v_b200.ops')
-    x3, x1 = rep['tf32x3'], rep['tf32']
-    assert x3['launches'] > 100 and x1['launches'] > 100, rep            # FIR / bias_act / tcgen05 launches of libsgv_b200, not a library fallback
-    # fp32-grade mode: image, logits and every sampled gradient agree with the CPU evaluation of the same unmodified modules
+    saved = conv2d_gradfix.enabled, torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
+    conv2d_gradfix.enabled = True                                   # training_loop.py:143
+    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
+    report = {}
+    try:
+        for mode in ('tf32x3', 'tf32'):
+            n0 = _lib.launch_count()
+            with precision.precision(mode):
+                got = run()
+            torch.cuda.synchronize()
+            report[mode] = dict(launches=_lib.launch_count() - n0, **{k: _rel(got[k], want[k]) for k in want})
+            report[mode]['cos'] = {k: float(torch.nn.functional.cosine_similarity(got[k].flatten(), want[k].flatten(), dim=0))
+                                   for k in want if k[1] == ':'}
+    finally:
+        conv2d_gradfix.enabled, torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = saved
+    x3, x1 = report['tf32x3'], report['tf32']
+    assert x3['launches'] > 100 and x1['launches'] > 100, report     # FIR / bias_act / tcgen05 launches of libsgv_b200, not a library fallback
+    # fp32-grade mode: image, logits and every sampled gradient agree with the reference's CPU evaluation
     assert x3['img'] < 1e-4 and x3['logits'] < 1e-4, x3
     for k, v in x3.items():
         if k[1:2] == ':':
@@ -120,103 +79,73 @@ def test_unmodified_reference_generator_and_discriminator_on_dropin_ops(tmp_path
     for k, cs in x1['cos'].items():
         if not k.endswith('bias'):
             assert cs > 0.99, (k, cs)
+    print('G + D at 64x64 vs the reference:', report)
 
 
-_LOSS_SCRIPT = r'''
-import sys, json, numpy as np, torch
-sys.path.insert(0, {root!r})
-from stylegan_v_b200.install import install_ops
-install_ops()
-from stylegan_v_b200 import _lib, precision
-from oracle import ref_loader, synthesis_ref as sr
-ref = ref_loader.load()
-from stylegan_v_b200.ops import conv2d_gradfix
-torch.backends.cudnn.allow_tf32 = False
-torch.backends.cuda.matmul.allow_tf32 = False
-
-# the reference draws its motion noise with torch.randn on the compute device (motion.py:83); route every draw through ONE CPU generator so that
-# the CPU and the CUDA evaluation see the same numbers (the reference code itself is untouched)
-_gen = torch.Generator()
-_randn = torch.randn
-def randn(*size, **kw):
-    dev = kw.pop('device', None)
-    kw.pop('generator', None)
-    out = _randn(*size, generator=_gen, **kw)
-    return out.to(dev) if dev is not None else out
-torch.randn = randn
-
-cfg = sr.SynthesisConfig(img_resolution=32, w_dim=64, channel_base=2048, channel_max=64, motion_z_dim=32, motion_v_dim=32, time_enc_dim=32)
-gcfg = ref_loader.to_cfg(cfg.reference_generator_cfg())
-dcfg = ref_loader.to_cfg(dict(sampling=dict(num_frames_per_video=3, max_num_frames=1024, type='random'), concat_res=16, num_frames_div_factor=2, dummy_c=False))
-torch.manual_seed(0)
-G = ref.networks.Generator(c_dim=0, w_dim=cfg.w_dim, img_resolution=32, img_channels=3, cfg=gcfg, mapping_kwargs=dict(num_layers=2),
-                           synthesis_kwargs=dict(channel_base=cfg.channel_base, channel_max=cfg.channel_max)).train()
-D = ref.networks.Discriminator(c_dim=0, img_resolution=32, img_channels=3, channel_base=2048, channel_max=64, cfg=dcfg,
-                               mapping_kwargs=dict(num_layers=2), epilogue_kwargs=dict(mbstd_group_size=2)).train()
-g = torch.Generator().manual_seed(1)
-B, Fr = 2, 3
-real = _randn(B, Fr, 3, 32, 32, generator=g).clamp(-1, 1)
-real_t = torch.tensor([[0.0, 4.0, 20.0], [30.0, 31.0, 33.0]])
-gen_t = torch.tensor([[2.0, 10.0, 11.0], [500.0, 516.0, 530.0]])
-z = _randn(B, cfg.w_dim, generator=g)
-c = torch.zeros(B, 0)
-PHASES = [('Gmain', 'G', 1), ('Dmain', 'D', 1), ('Dreg', 'D', 16)]
-
-
-def run(dev):
-    Gd, Dd = G.to(dev), D.to(dev)
-    loss = ref.loss.StyleGAN2Loss(cfg=None, device=dev, G_mapping=Gd.mapping, G_synthesis=Gd.synthesis, D=Dd, style_mixing_prob=0.0, r1_gamma=0.5, pl_weight=0.0)
-    w0 = Gd.mapping.w_avg.clone()
-    out = {{}}
-    for phase, which, gain in PHASES:
-        module = Gd if which == 'G' else Dd
-        Gd.requires_grad_(which == 'G'); Dd.requires_grad_(which == 'D')
+def loss_phase_grads(g, dev):
+    """Gmain, Dmain (with the motion noise the reference drew) and Dreg (gain 16) of the modules of loss_phases_32.npz on `dev`:
+    {phase:name: fixed sample of the gradient} for the weights the golden holds."""
+    G, D = M.seeded_modules(M.LOSS32_G, M.LOSS32_D)
+    assert M.param_sum(G, D) == pytest.approx(float(g['param_sum']), rel=1e-12), \
+        'the seeded initialisation of the modules changed: re-mint tests/golden/loss_phases_32.npz (python -m oracle.make_goldens gen_loss_phases_32)'
+    G, D = G.to(dev).train(), D.to(dev).train()
+    real = torch.from_numpy(g['real']).to(dev)
+    real = real.view(-1, *real.shape[2:])
+    real_t, gen_t, z = (torch.from_numpy(g[k]).to(dev) for k in ('real_t', 'gen_t', 'z'))
+    c = torch.zeros(len(z), 0, device=dev)
+    r1_gamma = json.loads(bytes(g['meta']).decode())['r1_gamma']
+    w0 = G.mapping.w_avg.clone()
+    out = {}
+    for phase in ('Gmain', 'Dmain', 'Dreg'):
+        module = G if phase == 'Gmain' else D
+        G.requires_grad_(module is G)
+        D.requires_grad_(module is D)
         for p in module.parameters():
             p.grad = None
-        _gen.manual_seed(100)
-        loss.accumulate_gradients(phase=phase, real_img=real.to(dev), real_c=c.to(dev), real_t=real_t.to(dev), gen_z=z.to(dev), gen_c=c.to(dev), gen_t=gen_t.to(dev), sync=True, gain=gain)
-        Gd.mapping.w_avg.copy_(w0)
-        for n, p in module.named_parameters():
-            if p.grad is not None and p.grad.numel() >= 64 and not n.endswith('bias'):
-                out[phase + ':' + n] = p.grad.double().cpu().clone()
+        if phase == 'Gmain':
+            ts.generator_main_loss(G, D, z, c, gen_t, motion_z=torch.from_numpy(g['motion_z:Gmain']).to(dev)).backward()
+        elif phase == 'Dmain':
+            a, b = ts.discriminator_main_loss(G, D, real, c, real_t, z, c, gen_t, motion_z=torch.from_numpy(g['motion_z:Dmain']).to(dev))
+            (a + b).backward()
+        else:
+            ts.discriminator_r1_loss(D, real, c, real_t, r1_gamma).mul(16).backward()
+        G.mapping.w_avg.copy_(w0)
+        P = dict(module.named_parameters())
+        for k in g.files:
+            if k.startswith(phase + ':') and not k.startswith('motion_z'):
+                out[k] = torch.from_numpy(M.sample(P[k.split(':', 1)[1]].grad))
     return out
 
 
-cpu = run(torch.device('cpu'))
-conv2d_gradfix.enabled = True
-n0 = _lib.launch_count()
-with precision.precision('tf32x3'):
-    gpu = run(torch.device('cuda', 0))
-torch.cuda.synchronize()
-rep = dict(launches=_lib.launch_count() - n0, grads=len(cpu))
-worst = {{}}
-for k in cpu:
-    a, b = gpu[k], cpu[k]
-    rel = float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
-    cs = float(torch.nn.functional.cosine_similarity(a.flatten(), b.flatten(), dim=0))
-    ph = k.split(':')[0]
-    w = worst.setdefault(ph, dict(rel=0.0, cos=1.0, n=0))
-    w['rel'] = max(w['rel'], rel); w['cos'] = min(w['cos'], cs); w['n'] += 1
-    if rel == w['rel']:
-        w['worst'] = k
-rep['worst'] = worst
-print('REPORT ' + json.dumps(rep))
-'''
-
-
-def test_unmodified_reference_loss_phases_on_dropin_ops():
-    """SURVEY §2 row 11: `StyleGAN2Loss` stays the reference's.  Its `accumulate_gradients` (loss.py:73-173) — Gmain, Dmain and the R1 phase, which
-    differentiates the discriminator twice — runs unmodified on the drop-in ops on cuda:0 (fp32-grade mode) and must reproduce the gradients of
-    its own CPU evaluation for every weight of the trained network."""
-    code = _LOSS_SCRIPT.format(root=ROOT)
-    env = dict(os.environ)
-    env.pop('SGV_PRECISION', None)
-    r = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, env=env, cwd=ROOT, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
-    rep = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith('REPORT ')][-1][len('REPORT '):])
-    assert rep['launches'] > 300 and rep['grads'] > 40, rep
-    for phase, w in rep['worst'].items():
-        # measured on the B200 (call M of round 2): worst max-norm error 1.7e-4 (Gmain) / 3.9e-4 (Dmain) / 7.7e-5 (Dreg), cosine 1 - 1e-8; bars 2e-3 / 0.9999
-        # (the fp32-grade mode; leaky-ReLU slope flips of a non-bit-equal forward are what the margin is for, tests/test_precision_gpu.py)
+def test_loss_phases_cuda_vs_reference_golden(cuda):
+    """SURVEY §2 row 11: the training loss follows the reference's `StyleGAN2Loss`.  Its Gmain, Dmain and R1 phases (the last differentiates
+    the discriminator twice) on cuda:0 in the fp32-grade mode must reproduce the reference's CPU gradients for every weight of the network."""
+    from stylegan_v_b200 import _lib, precision
+    from stylegan_v_b200.ops import conv2d_gradfix
+    g = np.load(f'{GOLDEN}/loss_phases_32.npz')
+    saved = conv2d_gradfix.enabled, torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
+    conv2d_gradfix.enabled = True
+    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
+    try:
+        n0 = _lib.launch_count()
+        with precision.precision('tf32x3'):
+            got = loss_phase_grads(g, cuda)
+        torch.cuda.synchronize()
+        launches = _lib.launch_count() - n0
+    finally:
+        conv2d_gradfix.enabled, torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = saved
+    assert launches > 300 and len(got) > 40, (launches, len(got))
+    worst = {}
+    for k, a in got.items():
+        b = torch.from_numpy(g[k]).double()
+        w = worst.setdefault(k.split(':')[0], dict(rel=0.0, cos=1.0, n=0))
+        rel = _rel(a, b)
+        if rel >= w['rel']:
+            w['rel'], w['worst'] = rel, k
+        w['cos'] = min(w['cos'], float(torch.nn.functional.cosine_similarity(a.flatten(), b.flatten(), dim=0)))
+        w['n'] += 1
+    for phase, w in worst.items():
+        # measured on the B200 with the reference modules on these kernels: worst max-norm error 1.7e-4 (Gmain) / 3.9e-4 (Dmain) / 7.7e-5 (Dreg),
+        # cosine 1 - 1e-8; the margin is for leaky-ReLU slope flips of a non-bit-equal forward (tests/test_precision_gpu.py)
         assert w['n'] > 5 and w['cos'] > 0.9999 and w['rel'] < 2e-3, (phase, w)
-    print('reference loss phases on the drop-in ops:', rep)
+    print('loss phases vs the reference:', worst)
